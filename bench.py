@@ -2,7 +2,12 @@
 """Headline benchmark: train-step sequences/sec of the recurrent forecaster (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--precision bf16|fp32]
-                    [--workload cfg2|cfg3|predict|batcher]
+                    [--workload cfg2|cfg3|predict|batcher] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (see dump_outputs).  The inputs depend only
+on the arguments, so two builds run with the same arguments can be compared output for output -- with a tolerance: runs
+of one build (cfg2, bf16, 20 steps, one B200 at its 1000 W power limit) wrote weights up to 4.4e-5 apart, not
+bit-identical.
 
 Default workload (what the driver runs) = BASELINE.json configs[1]: synthetic B=4096, T=48, F=32, O=16, 1-layer LSTM
 H=256, one full Train._train_step_point (fwd, weighted-MSE loss, BPTT, clip, Adadelta, MaxNorm).  N>1 = configs[3]:
@@ -75,6 +80,26 @@ def hbm_bytes_per_seq(w, predict=False, fused_head=False):
         bwd += T * (8.0 * H + 2.0 * H + (64.0 if fused_head else 2.0 * H) + 8.0 * H)
         wg += T * (2.0 * (I + H) + 8.0 * H)
     return fwd, bwd, wg
+
+
+DUMP_BYTES = 64 * 10 ** 6        # --dump-outputs writes at most this many bytes of array data in all
+
+
+def dump_outputs(d, arrays):
+    """Writes {name: float32 / float64 array} as d/<name>.npy ('/' in a name becomes '.').  Smallest first, each array
+    gets an equal share of the DUMP_BYTES still unused; one larger than its share keeps a fixed, seeded sample of its
+    rows (leading axis, in order), so every run with the same arguments stores the same elements."""
+    os.makedirs(d, exist_ok=True)
+    left = DUMP_BYTES
+    for i, name in enumerate(sorted(arrays, key=lambda n: arrays[n].nbytes)):
+        a = np.asarray(arrays[name])
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        share = left // (len(arrays) - i)
+        if a.nbytes > share:
+            keep = share // (a.nbytes // a.shape[0])
+            a = a[np.sort(np.random.default_rng(SEED).choice(a.shape[0], keep, replace=False))]
+        left -= a.nbytes
+        np.save(os.path.join(d, name.replace('/', '.') + '.npy'), a)
 
 
 def synthetic(batch, rng, w=None):
@@ -190,7 +215,7 @@ def run_reference(args, w, rank, world):
         return
     cores = os.cpu_count() or 1
     rows = args.cpu_rows or (w['B'] if w['mode'] == 'train' else 4096)
-    v, s_per_step, used = cpu_port_seq_per_s(w, rows, max(1, args.steps), cores, warm=args.warmup)   # W untimed steps, as asked
+    v, s_per_step, used = cpu_port_seq_per_s(w, rows, args.steps, cores, warm=args.warmup)   # W untimed steps, as asked
     full = rows == w['B']
     line = {
         'impl': 'reference', 'metric': w['metric'], 'value': v, 'unit': 'sequences/s', 'n_gpus': args.gpus,
@@ -264,11 +289,13 @@ def run_batcher(args, w, dev):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(args.steps):
-        gather_batch(tab, *idx[i % 8], **kw)
+        out = gather_batch(tab, *idx[i % 8], **kw)
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / args.steps
     launches = _native.load().lfmq_launch_count() - l0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {n: t.cpu().numpy() for n, t in zip(('x', 'y', 'seq_norm'), out)})
     written = B * Tn * (Fn + On) * 4 + B * 8
     read = B * Tn * (Fn + On) * 8 + B * 24
     peaks = load_peaks()
@@ -301,7 +328,13 @@ def main():
     ap.add_argument('--cpu-rows', type=int, default=0, help='windows per step of the CPU arm (default: all)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-loss-check', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step returned as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs applies to --impl native (the reference arm draws its own inputs)')
     args.warmup = max(args.warmup, 3)
     w = dict(WORKLOADS[args.workload])
     if args.batch:
@@ -391,13 +424,13 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(k):
-            fn(first + i)
+            last = fn(first + i)
         e1.record()
         sync()
         ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), last
 
     it = 0
     for _ in range(args.warmup):
@@ -410,17 +443,25 @@ def main():
     eng.profile(True)
     l0 = eng.launch_count
     t0 = time.perf_counter()
-    ms = timed(step_resident, args.steps, it)
+    ms, last = timed(step_resident, args.steps, it)
     t1 = time.perf_counter()
     launches = eng.launch_count - l0
     regions = eng.profile_read()
     eng.profile(False)
     it += args.steps
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        # copied now: the e2e steps below overwrite preds_dev and move the weights on
+        if predict:
+            outputs = {'preds': last.cpu().numpy()}
+        else:
+            outputs = {'loss_mse': last.cpu().numpy()}
+            outputs.update(('weights/' + spec[0], a) for spec, a in zip(eng.specs, eng.get_weights(trainable_only=False)))
     for _ in range(2):
         step_e2e(it)
         it += 1
-    ms_e2e = timed(step_e2e, args.steps, it)
+    ms_e2e, _ = timed(step_e2e, args.steps, it)
     if pipe is not None:
         pipe.finish()
     it += args.steps
@@ -432,7 +473,7 @@ def main():
         e2e = world * B * args.steps / (ms_e2e * 1e-3)
         peaks = load_peaks()
         peak_tf, peak_why = pick_peak(peaks, clocks)
-        k = max(args.steps, 1)
+        k = args.steps
         fwd_ms, bwd_ms, wg_ms, head_ms = (regions[n][0] / k for n in ('fwd', 'bwd', 'wgrad', 'head'))
         f_fwd, f_dg, f_wg = (f * B for f in flops_per_seq(w))
 
@@ -558,6 +599,8 @@ def main():
                                     'sample': '%d of %d windows per step, 2 steps after 1 warm-up (%.1f s); NumPy fp32 '
                                               'restatement of the reference step (TensorFlow unavailable); host has %d '
                                               'cores, `cores` = BLAS threads used' % (rows, B, 3 * s_step, cores)}
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

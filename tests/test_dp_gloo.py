@@ -107,8 +107,11 @@ def _cli_worker(rank, world, port, out_dir):
     dist.destroy_process_group()
 
 
-def test_cli_sharding_covers_every_global_batch_exactly_once(tmp_path):
+def test_cli_sharding_covers_every_global_batch_exactly_once(tmp_path, monkeypatch):
     world = 2
+    # the ranks take init_from_env's gloo branch on every machine: with CUDA visible it would give each rank a GPU of
+    # its own (NCCL), which a machine with fewer GPUs than ranks does not have
+    monkeypatch.setenv('CUDA_VISIBLE_DEVICES', '')
     mp.spawn(_cli_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
     per_rank = [np.load(str(tmp_path / ('cli%d.npy' % r)), allow_pickle=True) for r in range(world)]
     for bi, n in enumerate((7, 2, 1)):
