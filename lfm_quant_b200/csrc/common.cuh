@@ -58,10 +58,14 @@ inline bool debug_sync_on() {
 
 // Host side: launch with the programmatic-stream-serialization attribute (LFMQ_PDL=0 turns it off).  `attrs_extra` lets
 // the cluster kernels add their cluster dimension.
+inline bool pdl_on() {
+  static const bool on = !(getenv("LFMQ_PDL") && atoi(getenv("LFMQ_PDL")) == 0);
+  return on;
+}
 template <typename... KArgs, typename... Args>
 inline int launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, int cluster_x,
                       Args&&... args) {
-  static const bool on = !(getenv("LFMQ_PDL") && atoi(getenv("LFMQ_PDL")) == 0);
+  const bool on = pdl_on();
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;

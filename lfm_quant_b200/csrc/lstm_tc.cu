@@ -139,6 +139,10 @@ struct TcImpl {
   unsigned long long* progress = nullptr;      // device: steps completed by the backward kernel, counted across calls
   unsigned long long epoch = 0;
   int head_ctas = 0, head_wctas = 0;
+  // head beside the forward recurrence (head_paced_kernel; LFMQ_FWD_HEAD=0 turns it off, read when the handle is made)
+  bool fwd_head = false;
+  int sm_count = 0;
+  unsigned int* head_progress = nullptr;       // device [n_tiles_cap]: forward CTA-steps published per row tile
 };
 
 // =============================================================================================
@@ -209,7 +213,10 @@ struct FwdParams {
   __nv_bfloat16* cst;     // null: do not save
   const float* biasp;
   long long* trace;       // debug (LFMQ_TRACE_FWD=1): clock64 stamps of CTA 0, every third step
+  unsigned int* head_progress;   // null, or per row tile (HP_CSTRIDE apart): steps whose h_t is in global memory
 };
+
+constexpr int HP_CSTRIDE = 32;   // head_progress counters one 128-byte line apart
 
 #define FWD_TRACE(role, t, pt)                                                        \
   do {                                                                                \
@@ -309,9 +316,15 @@ __global__ void __launch_bounds__(FWD_THREADS, 1)
                                 b0 + 32 * (int)rank, 0xF);
             FWD_TRACE(0, t, 2);
             if (SAVE) mbar_arrive(&bars->tma_issued);
+            // h_{t-1} of all 4 CTAs is in global memory (acquired above): count it for the paced head.  A gpu-scope
+            // release, cumulative over the cluster barrier, from the one thread with a step of slack after it
+            if (p.head_progress && rank == 0)
+              red_release_gpu_add(p.head_progress + (it * p.n_clusters + cid) * HP_CSTRIDE, 1u);
           }
         }
         mbar_wait_cluster(&bars->h_written, (n_hw++) & 1);       // phase of step T-1 (keeps parities aligned)
+        if (p.head_progress && rank == 0)
+          red_release_gpu_add(p.head_progress + (it * p.n_clusters + cid) * HP_CSTRIDE, 1u);
       }
     }
   } else if (warp == 1) {
@@ -1261,6 +1274,332 @@ __global__ void head_fold_kernel(int O, float* __restrict__ gWo, const float* __
   ggamma[j] = iv * (sg - mean[j] * db);
 }
 
+// ---------------------------------------------------------------------------------------------
+// Training head beside the forward recurrence (dropout off, one tile iteration of the recurrence).  Launched as the
+// programmatic dependent of lstm_fwd_tc_kernel<true>, whose CTAs all trigger it right after their own wait: the grid
+// is dispatched once the whole recurrence is resident and lands on the SMs it leaves idle (the shared memory below
+// cannot fit beside a forward CTA, and only one fits per SM).  CTA j owns the row tiles bt = j, j+G, .. and walks
+// (t, tile) in t order; the h_t tile is fetched once the forward has counted step t on the tile's counter.  Per tile it does exactly what head_tc_kernel<true> does: pred = h WoTp + bop on tcgen05, the masked
+// weighted-MSE terms, the bf16 dpred tile TMA-stored for the backward recurrence, h^T dpred accumulated in TMEM.
+// Loss sums, colsum(dpred) and h^T dpred go to fixed per-CTA slots, summed in a fixed order: the results depend only
+// on the inputs.  The forward never waits on this kernel.
+//   warp 0: h tiles (TMA, 3-stage ring), warp 1: MMAs + dpred store, warps 2-5: one row per thread.
+// ---------------------------------------------------------------------------------------------
+constexpr int HP_STAGES = 3;
+constexpr uint32_t HP_H = 0;                                   // HP_STAGES x 4 k-blocks x [128 x 128 B]
+constexpr uint32_t HP_WOT = HP_STAGES * 65536;                 // 4 k-blocks x [16 x 128 B]
+constexpr uint32_t HP_DP = HP_WOT + 8192;                      // 2 x [128 x 64 B]
+constexpr uint32_t HP_BARS = HP_DP + 2 * 8192;
+constexpr int HP_SMEM = HP_BARS + 256 + 1024;
+constexpr int HP_THREADS = 192;
+constexpr int HP_PART = 3 + TC_OPAD;                           // s0 s1 s2 | colsum(dpred), per CTA
+constexpr int HP_TRACE_UNITS = 128;                            // LFMQ_TRACE_HEAD: stamps of CTA 0's first units
+constexpr int SM_SMEM_BYTES = 233472;                          // shared memory per SM (228 KB)
+static_assert(HP_SMEM + FWD_SMEM > SM_SMEM_BYTES, "a paced head CTA must not fit beside a forward CTA");
+static_assert(2 * HP_SMEM > SM_SMEM_BYTES, "one paced head CTA per SM");
+
+struct HpBars {
+  uint64_t wt_full, w_done;
+  uint64_t h_full[HP_STAGES], h_empty[HP_STAGES];
+  uint64_t pred_full[2], acc_free[2], dp_full[2], dp_free[2];
+  uint32_t tmem_base;
+};
+
+__global__ void __launch_bounds__(HP_THREADS, 1)
+    head_paced_kernel(HeadParams p, HeadTcWeights w, const __grid_constant__ CUtensorMap tm_h,
+                      const __grid_constant__ CUtensorMap tm_wot, const __grid_constant__ CUtensorMap tm_dpb, int n_btiles,
+                      int n_tiles_cap, unsigned int* __restrict__ progress, float* __restrict__ wpartial,
+                      float* __restrict__ hpart) {
+  // No griddepcontrol.wait before the loop: this grid runs beside the forward recurrence.  WoTp, bop, the denominators
+  // and y were written by grids that the forward's own wait has already seen complete (the forward triggers this grid
+  // only after that wait); h_t is acquired through progress[].  The backward may be dispatched at once: it cannot get
+  // an SM before forward CTAs leave, and its own wait is on this grid, which ends only after the forward (see below).
+  griddep_launch_dependents();
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  HpBars* bars = reinterpret_cast<HpBars*>(smem + HP_BARS);
+  __shared__ float red_s[4][HP_PART];
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int G = gridDim.x, j0 = blockIdx.x;
+  const int nk = (n_btiles - j0 + G - 1) / G;       // row tiles of this CTA (G <= n_btiles, so >= 1)
+  const int N = p.T * nk;                           // units (t, k), t-major
+  long long* trc = (p.trace && blockIdx.x == 0) ? p.trace : nullptr;
+  if (trc && tid == 0) {
+    trc[0] = (long long)ld_acquire_gpu(progress + j0 * HP_CSTRIDE);   // forward steps already counted at the start
+    trc[1] = (long long)globaltimer_ns();
+  }
+  for (int i = tid; i < 2 * 8192 / 16; i += HP_THREADS) reinterpret_cast<uint4*>(smem + HP_DP)[i] = make_uint4(0, 0, 0, 0);
+  if (tid == 0) {
+    mbar_init(&bars->wt_full, 1);
+    mbar_init(&bars->w_done, 1);
+    for (int s = 0; s < HP_STAGES; ++s) {
+      mbar_init(&bars->h_full[s], 1);
+      mbar_init(&bars->h_empty[s], 1);
+    }
+    for (int a = 0; a < 2; ++a) {
+      mbar_init(&bars->pred_full[a], 1);
+      mbar_init(&bars->acc_free[a], 128);
+      mbar_init(&bars->dp_full[a], 128);
+      mbar_init(&bars->dp_free[a], 1);
+    }
+    fence_mbar_init();
+  }
+  if (warp == 0) tmem_alloc(&bars->tmem_base, 64);
+  fence_proxy_async_smem();
+  tcgen05_fence_before();
+  __syncthreads();
+  tcgen05_fence_after();
+  const uint32_t tmem = bars->tmem_base;
+  const uint32_t acc_p = tmem;             // 2 x 16 columns: pred of alternate units
+  const uint32_t acc_w = tmem + 32;        // 2 x 16 columns: sum over this CTA's units of h^T dpred (rows = hidden unit)
+
+  if (warp == 0) {
+    if (lane == 0) {
+      mbar_arrive_expect_tx(&bars->wt_full, 8192);
+      for (int kb = 0; kb < 4; ++kb) tma_load_2d(smem + HP_WOT + kb * 2048, &tm_wot, &bars->wt_full, kb * 64, 0);
+      for (int n = 0; n < N; ++n) {
+        const int t = n / nk, bt = j0 + (n % nk) * G, s = n % HP_STAGES;
+        if (n >= HP_STAGES) mbar_wait(&bars->h_empty[s], ((n / HP_STAGES) - 1) & 1);
+        const long long spin0 = clock64();
+        while (ld_acquire_gpu(progress + bt * HP_CSTRIDE) < (unsigned int)(t + 1)) {
+          // the forward is resident before this grid starts and never waits on it; should the count never come, fail
+          // the launch after ~2 s instead of hanging the device
+          if (clock64() - spin0 > 4000000000LL) __trap();
+        }
+        fence_proxy_async_global();
+        if (trc && n < HP_TRACE_UNITS) trc[2 + 2 * n] = (long long)globaltimer_ns();
+        mbar_arrive_expect_tx(&bars->h_full[s], 65536);
+        for (int kb = 0; kb < 4; ++kb)
+          tma_load_2d(smem + HP_H + s * 65536 + kb * 16384, &tm_h, &bars->h_full[s], (t + 1) * TC_XH_LD + kb * 64, bt * 128);
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {
+      const uint32_t idesc_p = make_idesc_bf16(128, 16, false, false);
+      const uint32_t idesc_w = make_idesc_bf16(128, 16, true, true);
+      mbar_wait(&bars->wt_full, 0);
+      for (int n = 0; n <= N; ++n) {
+        if (n < N) {        // pred of unit n ...
+          const int s = n % HP_STAGES, a = n & 1;
+          mbar_wait(&bars->h_full[s], (n / HP_STAGES) & 1);
+          if (n >= 2) mbar_wait(&bars->acc_free[a], ((n >> 1) - 1) & 1);
+          tcgen05_fence_after();
+#pragma unroll
+          for (int kb = 0; kb < 4; ++kb)
+#pragma unroll
+            for (int k16 = 0; k16 < 4; ++k16) {
+              const uint64_t da = make_smem_desc(smem_u32(smem + HP_H + s * 65536 + kb * 16384) + k16 * 32, 0, 1024,
+                                                 LAYOUT_SW128);
+              const uint64_t db = make_smem_desc(smem_u32(smem + HP_WOT + kb * 2048) + k16 * 32, 0, 1024, LAYOUT_SW128);
+              umma_f16(acc_p + a * 16, da, db, idesc_p, (kb | k16) != 0);
+            }
+          umma_commit(&bars->pred_full[a]);
+        }
+        if (n >= 1) {       // ... while the rows finish unit n-1: its dpred tile to HBM and into h^T dpred
+          const int u = n - 1, s = u % HP_STAGES, d = u & 1;
+          const int t = u / nk, bt = j0 + (u % nk) * G;
+          mbar_wait(&bars->dp_full[d], (u >> 1) & 1);
+          tcgen05_fence_after();
+          tma_store_2d(&tm_dpb, smem + HP_DP + d * 8192, 0, (t * n_tiles_cap + bt) * 128);
+          bulk_commit_group();
+#pragma unroll
+          for (int mb = 0; mb < 2; ++mb)
+#pragma unroll
+            for (int k16 = 0; k16 < 8; ++k16) {
+              const uint64_t wa = make_smem_desc(smem_u32(smem + HP_H + s * 65536 + 2 * mb * 16384) + k16 * 2048, 16384,
+                                                 1024, LAYOUT_SW128);
+              const uint64_t wb = make_smem_desc(smem_u32(smem + HP_DP + d * 8192) + k16 * 1024, 0, 512, LAYOUT_SW64);
+              umma_f16(acc_w + mb * 16, wa, wb, idesc_w, (u > 0 || k16 > 0) ? 1u : 0u);
+            }
+          umma_commit(&bars->h_empty[s]);     // both MMAs of unit u are done with the h stage
+          bulk_wait_group_read0();            // the store has read the dpred tile ...
+          umma_commit(&bars->dp_free[d]);     // ... and the h^T dpred MMAs are done with it
+          if (trc && u < HP_TRACE_UNITS) trc[3 + 2 * u] = (long long)globaltimer_ns();
+        }
+      }
+      umma_commit(&bars->w_done);
+      bulk_wait_group0();
+    }
+  } else {
+    const int wq = warp & 3;                // TMEM lane quadrant of this warp
+    const int mrow = wq * 32 + lane;        // row this thread can reach in TMEM == row it owns
+    const uint32_t lane_addr = (uint32_t)(wq * 32) << 16;
+    const float Bg = p.denom[0], Mg = p.denom[1];
+    const float c_all = (1.f - p.p1) * (1.f - p.p2) / ((float)p.O * Mg);
+    const float c_last = (1.f - p.p1) * p.p2 / (Bg * (float)p.O);
+    const float c_tar = p.p1 / Bg;
+    float bop[TC_OPAD];
+#pragma unroll
+    for (int k = 0; k < TC_OPAD; ++k) bop[k] = w.bop[k];
+    float s0 = 0.f, s1 = 0.f, s2 = 0.f;
+    float accbo[TC_OPAD];
+#pragma unroll
+    for (int k = 0; k < TC_OPAD; ++k) accbo[k] = 0.f;
+    // y of a unit does not depend on the forward: fetched one unit ahead
+    auto load_y = [&](int n, float* yv) {
+      const int t = n / nk, bt = j0 + (n % nk) * G;
+      const long b = (long)bt * 128 + mrow;
+#pragma unroll
+      for (int k = 0; k < TC_OPAD; ++k) yv[k] = 0.f;
+      if (b < p.B) {
+        const long r = b * p.T + t;
+#pragma unroll
+        for (int k = 0; k < TC_OPAD; ++k)
+          if (k < p.O) yv[k] = p.y[r * p.O + k];
+      }
+    };
+    float yt[TC_OPAD];
+    load_y(0, yt);
+    for (int n = 0; n < N; ++n) {
+      const int t = n / nk, bt = j0 + (n % nk) * G, a = n & 1;
+      const bool valid = (long)bt * 128 + mrow < p.B;
+      float yn[TC_OPAD];
+      if (n + 1 < N) load_y(n + 1, yn);
+      mbar_wait(&bars->pred_full[a], (n >> 1) & 1);
+      tcgen05_fence_after();
+      uint32_t pv[16];
+      tmem_ld_32x32b_x16(acc_p + a * 16 + lane_addr, pv);
+      tmem_ld_wait();
+      tcgen05_fence_before();
+      mbar_arrive(&bars->acc_free[a]);
+      bool any = false;
+#pragma unroll
+      for (int k = 0; k < TC_OPAD; ++k) any |= (yt[k] != 0.0f);          // losses.py:72
+      const float mk = (any && valid) ? 1.f : 0.f;
+      const bool last = (t == p.T - 1);
+      float dp[TC_OPAD];
+#pragma unroll
+      for (int k = 0; k < TC_OPAD; ++k) {
+        const float pr = __uint_as_float(pv[k]) + bop[k];
+        const float d = (k < p.O && valid) ? (pr * mk - yt[k]) : 0.f;  // losses.py:75
+        const float d2 = d * d;
+        s2 += d2;
+        float coef = c_all;
+        if (last) {
+          s1 += d2;
+          coef += c_last;
+          if (k == p.target_idx) {
+            s0 += d2;
+            coef += c_tar;
+          }
+        }
+        dp[k] = 2.f * d * coef * mk;
+        accbo[k] += dp[k];
+      }
+      // dpred row -> [128 x 64 B] SWIZZLE_64B tile: chunk c of row m at m*64 + ((c ^ ((m>>1)&3)) << 4)
+      if (n >= 2) mbar_wait(&bars->dp_free[a], ((n >> 1) - 1) & 1);
+      uint8_t* drow = smem + HP_DP + a * 8192 + mrow * 64;
+      const int s64 = (mrow >> 1) & 3;
+      *reinterpret_cast<uint4*>(drow + ((0 ^ s64) << 4)) =
+          make_uint4(pack_bf16x2(dp[0], dp[1]), pack_bf16x2(dp[2], dp[3]), pack_bf16x2(dp[4], dp[5]), pack_bf16x2(dp[6], dp[7]));
+      *reinterpret_cast<uint4*>(drow + ((1 ^ s64) << 4)) =
+          make_uint4(pack_bf16x2(dp[8], dp[9]), pack_bf16x2(dp[10], dp[11]), pack_bf16x2(dp[12], dp[13]), pack_bf16x2(dp[14], dp[15]));
+      fence_proxy_async_smem();
+      mbar_arrive(&bars->dp_full[a]);
+#pragma unroll
+      for (int k = 0; k < TC_OPAD; ++k) yt[k] = yn[k];
+    }
+    s0 = warp_sum(s0); s1 = warp_sum(s1); s2 = warp_sum(s2);
+#pragma unroll
+    for (int k = 0; k < TC_OPAD; ++k) accbo[k] = warp_sum(accbo[k]);
+    if (lane == 0) {
+      red_s[wq][0] = s0; red_s[wq][1] = s1; red_s[wq][2] = s2;
+#pragma unroll
+      for (int k = 0; k < TC_OPAD; ++k) red_s[wq][3 + k] = accbo[k];
+    }
+    // this CTA's h^T dpred: TMEM lane = hidden unit (mod 128), 16 columns per 128-unit block
+    float* wp = wpartial + (long)blockIdx.x * HWG_PART;
+    mbar_wait(&bars->w_done, 0);
+    tcgen05_fence_after();
+#pragma unroll
+    for (int mb = 0; mb < 2; ++mb) {
+      uint32_t v[16];
+      tmem_ld_32x32b_x16(acc_w + lane_addr + mb * 16, v);
+      tmem_ld_wait();
+      float* o = wp + (mb * 128 + mrow) * TC_OPAD;
+#pragma unroll
+      for (int k4 = 0; k4 < 16; k4 += 4)
+        *reinterpret_cast<float4*>(o + k4) = make_float4(__uint_as_float(v[k4]), __uint_as_float(v[k4 + 1]),
+                                                         __uint_as_float(v[k4 + 2]), __uint_as_float(v[k4 + 3]));
+    }
+  }
+  __syncwarp();
+  tcgen05_fence_before();
+  __syncthreads();
+  if (tid < HP_PART) hpart[(long)blockIdx.x * HP_PART + tid] = ((red_s[0][tid] + red_s[1][tid]) + red_s[2][tid]) + red_s[3][tid];
+  if (warp == 0) tmem_dealloc(tmem, 64);
+  // The forward is complete past this wait, so (1) its counts on this CTA's tiles are final and can be reset for the
+  // next call -- only this CTA reads them, and the next forward is ordered after this grid -- and (2) the next kernel
+  // (the backward, whose wait is on this grid) sees the forward's deferred saved-state stores.
+  griddep_wait();
+  for (int bt = j0 + tid * G; bt < n_btiles; bt += G * HP_THREADS) progress[bt * HP_CSTRIDE] = 0u;
+}
+
+// What the paced head leaves per CTA, reduced and folded into the head gradients and the loss by the launch that also
+// reduces the weight gradient (wgrad_head_reduce_kernel).
+struct HeadFoldArgs {
+  int G, O;
+  const float* hpart;          // [G][HP_PART]
+  const float* wpart;          // [G][256 * 16]  h^T dpred
+  const float* denom;
+  float p1, p2, eps;
+  const float *Wo, *gamma, *beta, *mean, *var;
+  float *gWo, *gbo, *ggamma, *gbeta, *out2;
+};
+constexpr int HF_UNITS = 16;                            // hidden units per fold block
+constexpr int HF_BLOCKS = TC_H / HF_UNITS + 1;          // + one block for the loss
+
+// Block bid < TC_H / HF_UNITS: sums (in double, CTA order) h^T dpred for its 16 hidden units and colsum(dpred), then
+// the fold of head_fold_kernel; block TC_H / HF_UNITS: the loss of head_reduce_kernel.  256 threads.
+__device__ __forceinline__ void head_fold_body(int bid, const HeadFoldArgs& a) {
+  __shared__ float cs_s[TC_OPAD];
+  __shared__ float g_s[HF_UNITS][TC_OPAD];
+  __shared__ double l_s[3];
+  const int tid = threadIdx.x;
+  if (bid == TC_H / HF_UNITS) {
+    if (tid < 3) {
+      double s = 0.0;
+      for (int c = 0; c < a.G; ++c) s += a.hpart[(long)c * HP_PART + tid];
+      l_s[tid] = s;
+    }
+    __syncthreads();
+    if (tid == 0) {
+      const double Bg = a.denom[0], Mg = a.denom[1];
+      const double mse0 = l_s[0] / Bg, mse1 = l_s[1] / (Bg * a.O), mse2 = l_s[2] / (Mg * a.O);
+      a.out2[0] = (float)(a.p1 * mse0 + (1.0 - a.p1) * (a.p2 * mse1 + (1.0 - a.p2) * mse2));
+      a.out2[1] = (float)mse0;
+    }
+    return;
+  }
+  if (tid < TC_OPAD) {
+    double s = 0.0;
+    for (int c = 0; c < a.G; ++c) s += a.hpart[(long)c * HP_PART + 3 + tid];
+    cs_s[tid] = (float)s;
+    if (bid == 0 && tid < a.O) a.gbo[tid] = (float)s;
+  }
+  const int jl = tid / TC_OPAD, k = tid % TC_OPAD, j0 = bid * HF_UNITS;
+  {
+    double s = 0.0;
+    for (int c = 0; c < a.G; ++c) s += a.wpart[(long)c * HWG_PART + (j0 + jl) * TC_OPAD + k];
+    g_s[jl][k] = (float)s;
+  }
+  __syncthreads();
+  if (tid < HF_UNITS) {
+    const int j = j0 + tid;
+    const float iv = 1.0f / sqrtf(a.var[j] + a.eps);
+    const float aa = a.gamma[j] * iv, cc = a.beta[j] - a.gamma[j] * a.mean[j] * iv;
+    float db = 0.f, sg = 0.f;
+    for (int q = 0; q < a.O; ++q) {
+      const float wv = a.Wo[j * a.O + q], g = g_s[tid][q], cs = cs_s[q];
+      db = fmaf(wv, cs, db);
+      sg = fmaf(wv, g, sg);
+      a.gWo[j * a.O + q] = fmaf(aa, g, cc * cs);
+    }
+    a.gbeta[j] = db;
+    a.ggamma[j] = iv * (sg - a.mean[j] * db);
+  }
+}
+
 // =============================================================================================
 // Host side
 // =============================================================================================
@@ -1353,6 +1692,7 @@ int tc_init(TcState& st, const lfmq_config& c) {
     return rc;
   LFMQ_CUDA_CHECK(cudaFuncSetAttribute(head_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, HT_SMEM));
   LFMQ_CUDA_CHECK(cudaFuncSetAttribute(head_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, HT_SMEM));
+  LFMQ_CUDA_CHECK(cudaFuncSetAttribute(head_paced_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, HP_SMEM));
   LFMQ_CUDA_CHECK(cudaFuncSetAttribute(head_rows_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, HROWS_SMEM));
   LFMQ_CUDA_CHECK(cudaFuncSetAttribute(head_rows_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, HROWS_SMEM));
   if ((rc = make_map_2d(&m.tm_u, m.Up, TC_H, 4 * TC_H, TC_H * 2, 64, 256, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
@@ -1378,6 +1718,15 @@ int tc_init(TcState& st, const lfmq_config& c) {
     return LFMQ_ERR_UNSUPPORTED;
   }
   m.max_clusters = nclusters;
+  int dev = 0;
+  LFMQ_CUDA_CHECK(cudaGetDevice(&dev));
+  LFMQ_CUDA_CHECK(cudaDeviceGetAttribute(&m.sm_count, cudaDevAttrMultiProcessorCount, dev));
+  m.fwd_head = !(getenv("LFMQ_FWD_HEAD") && atoi(getenv("LFMQ_FWD_HEAD")) == 0);
+  if (m.dpb && m.fwd_head) {
+    const size_t n = (size_t)((m.maxB + 127) / 128) * HP_CSTRIDE;
+    LFMQ_CUDA_CHECK(cudaMalloc(&m.head_progress, n * sizeof(unsigned int)));
+    LFMQ_CUDA_CHECK(cudaMemset(m.head_progress, 0, n * sizeof(unsigned int)));
+  }
   m.enabled = true;
   st.weights_dirty = 1;
   return 0;
@@ -1391,6 +1740,7 @@ void tc_destroy(TcState& st) {
     cudaStreamDestroy(st.impl->side);
     cudaFree(st.impl->progress);
   }
+  if (st.impl && st.impl->head_progress) cudaFree(st.impl->head_progress);
   delete st.impl;
   st.impl = nullptr;
 }
@@ -1413,7 +1763,7 @@ static int tc_pack_weights(TcState& st, const float* params, cudaStream_t s) {
   return 0;
 }
 
-static int tc_run_recurrence(TcState& st, const float* x, int B, bool save, cudaStream_t s) {
+static int tc_run_recurrence(TcState& st, const float* x, int B, bool save, unsigned int* head_progress, cudaStream_t s) {
   TcImpl& m = *st.impl;
   const long bt = (long)B * m.T * 5;
   if (int rc = launch_pdl(xh_fill_x_kernel, dim3((int)((bt + 255) / 256)), dim3(256), 0, s, 1, B, m.T, m.I, x, m.xh)) return rc;
@@ -1428,6 +1778,7 @@ static int tc_run_recurrence(TcState& st, const float* x, int B, bool save, cuda
   p.gates = save ? m.gates : nullptr;
   p.cst = save ? m.cst : nullptr;
   p.biasp = m.biasp;
+  p.head_progress = head_progress;
   static long long* trace_dev = nullptr;
   static const bool want_trace = getenv("LFMQ_TRACE_FWD") != nullptr;
   if (want_trace && !trace_dev) {
@@ -1566,7 +1917,7 @@ int tc_forward(TcState& st, const lfmq_config& c, const float* params, const flo
   int rc;
   if ((rc = tc_pack_weights(st, params, s))) return rc;
   st.prof->begin(LFMQ_REGION_FWD, s);
-  if ((rc = tc_run_recurrence(st, x, B, save, s))) return rc;
+  if ((rc = tc_run_recurrence(st, x, B, save, nullptr, s))) return rc;
   st.prof->end(LFMQ_REGION_FWD, s);
   if (preds) {
     st.prof->begin(LFMQ_REGION_HEAD, s);
@@ -1577,7 +1928,7 @@ int tc_forward(TcState& st, const lfmq_config& c, const float* params, const flo
 }
 
 int tc_backward_impl(TcState& st, const lfmq_config& c, const float* params, float* grads, int B, bool fused,
-                     cudaStream_t s);
+                     const HeadFoldArgs* hf, cudaStream_t s);
 
 int tc_backward(TcState& st, const lfmq_config& c, const float* params, float* grads, const float* x, const float* y,
                 int B, int64_t row0, int64_t step, const float* denom, float* tail, cudaStream_t s) {
@@ -1585,16 +1936,68 @@ int tc_backward(TcState& st, const lfmq_config& c, const float* params, float* g
     LFMQ_SET_ERR("bf16 path not initialised");
     return LFMQ_ERR_UNSUPPORTED;
   }
+  TcImpl& m = *st.impl;
   int rc;
   if ((rc = tc_pack_weights(st, params, s))) return rc;
+  const bool dropout = c.train && c.dropout > 0.f;
+  // The head runs beside the forward recurrence on the SMs it leaves idle when: the tensor-core head (no dropout), one
+  // tile iteration of the recurrence (every cluster resident, so the head cannot take a forward cluster's SMs), enough
+  // idle SMs, and programmatic dependent launch (what dispatches the head only once the recurrence is resident).
+  const int n_tiles = (B + 127) / 128;
+  const int idle = m.sm_count - TC_NC * n_tiles;
+  const bool paced = m.head_progress && !dropout && n_tiles <= m.max_clusters && idle >= 8 && pdl_on();
+  static long long* ptrace = nullptr;
+  static const bool want_ptrace = getenv("LFMQ_TRACE_HEAD") != nullptr;
+  if (paced && want_ptrace) {
+    const size_t ntr = 2 + 2 * HP_TRACE_UNITS;
+    if (!ptrace) LFMQ_CUDA_CHECK(cudaMalloc(&ptrace, ntr * sizeof(long long)));
+    LFMQ_CUDA_CHECK(cudaMemsetAsync(ptrace, 0, ntr * sizeof(long long), s));
+  }
   st.prof->begin(LFMQ_REGION_FWD, s);
-  if ((rc = tc_run_recurrence(st, x, B, true, s))) return rc;
-  st.prof->end(LFMQ_REGION_FWD, s);
-  st.prof->begin(LFMQ_REGION_HEAD, s);
-  if ((rc = tc_run_head(st, c, params, grads, y, B, row0, step, denom, nullptr, tail, true, s))) return rc;
-  st.prof->end(LFMQ_REGION_HEAD, s);
+  if ((rc = tc_run_recurrence(st, x, B, true, paced ? m.head_progress : nullptr, s))) return rc;
+  HeadFoldArgs hf;
+  if (paced) {
+    // nothing between the two launches (no event, no copy): the head must be dispatched while the recurrence runs
+    const int G = idle < n_tiles ? idle : n_tiles;
+    HeadParams h = {};
+    h.B = B; h.T = m.T; h.O = m.O; h.target_idx = c.target_idx; h.train = 1;
+    h.y = y; h.denom = denom; h.p1 = c.target_lambda; h.p2 = c.rnn_lambda;
+    h.trace = want_ptrace ? ptrace : nullptr;
+    HeadTcWeights hw;
+    hw.WoTp = m.WoTp; hw.bop = m.bop;
+    if ((rc = launch_pdl(head_paced_kernel, dim3(G), dim3(HP_THREADS), HP_SMEM, s, 1, h, hw, m.tm_h128, m.tm_wot, m.tm_dpb,
+                         n_tiles, (m.maxB + 127) / 128, m.head_progress, m.head_wpart, m.head_part)))
+      return rc;
+    st.prof->end(LFMQ_REGION_FWD, s);
+    if (want_ptrace) {
+      // CTA 0: forward CTA-steps counted on its first tile when it started, then per unit (t, tile) the global-timer
+      // time at which h_t was there and at which the unit was finished, relative to the first
+      long long tr[2 + 2 * HP_TRACE_UNITS];
+      LFMQ_CUDA_CHECK(cudaStreamSynchronize(s));
+      LFMQ_CUDA_CHECK(cudaMemcpy(tr, ptrace, sizeof(tr), cudaMemcpyDeviceToHost));
+      const int nk = (n_tiles + G - 1) / G, nu = m.T * nk < HP_TRACE_UNITS ? m.T * nk : HP_TRACE_UNITS;
+      const long long t0 = tr[2];
+      fprintf(stderr, "[ptrace] G=%d units/CTA0=%d forward counts at start=%lld start=%lld ns\n", G, m.T * nk, tr[0],
+              tr[1] - t0);
+      for (int u = 0; u < nu; ++u)
+        fprintf(stderr, "[ptrace] unit %3d t=%2d ready %8lld done %8lld lag %6lld ns\n", u, u / nk, tr[2 + 2 * u] - t0,
+                tr[3 + 2 * u] - t0, tr[3 + 2 * u] - tr[2 + 2 * u]);
+    }
+    hf.G = G; hf.O = m.O;
+    hf.hpart = m.head_part; hf.wpart = m.head_wpart;
+    hf.denom = denom; hf.p1 = c.target_lambda; hf.p2 = c.rnn_lambda; hf.eps = c.bn_epsilon;
+    hf.Wo = params + m.oWo; hf.gamma = params + m.ogamma; hf.beta = params + m.obeta; hf.mean = params + m.omean;
+    hf.var = params + m.ovar;
+    hf.gWo = grads + m.oWo; hf.gbo = grads + m.obo; hf.ggamma = grads + m.ogamma; hf.gbeta = grads + m.obeta;
+    hf.out2 = tail;
+  } else {
+    st.prof->end(LFMQ_REGION_FWD, s);
+    st.prof->begin(LFMQ_REGION_HEAD, s);
+    if ((rc = tc_run_head(st, c, params, grads, y, B, row0, step, denom, nullptr, tail, true, s))) return rc;
+    st.prof->end(LFMQ_REGION_HEAD, s);
+  }
   // the tensor-core head (no dropout) leaves dLoss/dpred tiles for the backward kernel to expand on its own MMAs
-  return tc_backward_impl(st, c, params, grads, B, /*fused=*/!(c.train && c.dropout > 0.f), s);
+  return tc_backward_impl(st, c, params, grads, B, /*fused=*/!dropout, paced ? &hf : nullptr, s);
 }
 
 }  // namespace lfmq
@@ -2212,10 +2615,9 @@ __global__ void __launch_bounds__(WG_THREADS, 1)
 
 // Sums the K-split partials and scatters D rows into dU / dW / db of the flat gradient vector.  D's columns are in
 // dz's order [16-unit block][gate][16]; the gradients want gate-major columns g*H + unit.
-__global__ void wgrad_reduce_kernel(int S, int I, const float* __restrict__ partial, float* __restrict__ gU,
-                                    float* __restrict__ gW, float* __restrict__ gb) {
-  pdl_sync();
-  const long idx = (long)blockIdx.x * blockDim.x + threadIdx.x;
+__device__ __forceinline__ void wgrad_reduce_body(int bid, int S, int I, const float* __restrict__ partial,
+                                                  float* __restrict__ gU, float* __restrict__ gW, float* __restrict__ gb) {
+  const long idx = (long)bid * blockDim.x + threadIdx.x;
   if (idx >= (long)384 * 1024) return;
   const int row = (int)(idx / 1024), np = (int)(idx % 1024);
   const int n = ((np % 64) / 16) * TC_H + (np / 64) * 16 + (np % 16);
@@ -2227,6 +2629,26 @@ __global__ void wgrad_reduce_kernel(int S, int I, const float* __restrict__ part
   float s = 0.f;
   for (int z = 0; z < S; ++z) s += partial[(long)z * 384 * 1024 + idx];
   *dst = s;
+}
+
+constexpr int WGR_BLOCKS = (384 * 1024 + 255) / 256;
+
+__global__ void __launch_bounds__(256) wgrad_reduce_kernel(int S, int I, const float* __restrict__ partial,
+                                                           float* __restrict__ gU, float* __restrict__ gW,
+                                                           float* __restrict__ gb) {
+  pdl_sync();
+  wgrad_reduce_body(blockIdx.x, S, I, partial, gU, gW, gb);
+}
+
+// With the paced head: blocks [0, HF_BLOCKS) reduce and fold the head's partials (head_fold_body; first, because
+// their serial sums over the head CTAs take longer than a reduce block), the rest the weight gradient.  Off the path
+// between the two recurrences.
+__global__ void __launch_bounds__(256) wgrad_head_reduce_kernel(int S, int I, const float* __restrict__ partial,
+                                                                float* __restrict__ gU, float* __restrict__ gW,
+                                                                float* __restrict__ gb, HeadFoldArgs hf) {
+  pdl_sync();
+  if (blockIdx.x < HF_BLOCKS) head_fold_body(blockIdx.x, hf);
+  else wgrad_reduce_body(blockIdx.x - HF_BLOCKS, S, I, partial, gU, gW, gb);
 }
 
 // Runs beside lstm_bwd_tc_kernel on the SMs it leaves idle: pulls the saved gates / cell states of the time step that
@@ -2270,7 +2692,7 @@ __global__ void __launch_bounds__(128) bwd_prefetch_kernel(const __nv_bfloat16* 
 }
 
 int tc_backward_impl(TcState& st, const lfmq_config& c, const float* params, float* grads, int B, bool fused,
-                     cudaStream_t s) {
+                     const HeadFoldArgs* hf, cudaStream_t s) {
   TcImpl& m = *st.impl;
   int rc;
   if (!m.bwd_ready) {
@@ -2391,9 +2813,15 @@ int tc_backward_impl(TcState& st, const lfmq_config& c, const float* params, flo
   S = (wp.n_kblocks + wp.kb_per_split - 1) / wp.kb_per_split;
   wp.partial = m.wg_part;
   if ((rc = launch_pdl(wgrad_tc_kernel, dim3(3, 4, S), dim3(WG_THREADS), WG_SMEM, s, 1, wp, tm_a, tm_b))) return rc;
-  if ((rc = launch_pdl(wgrad_reduce_kernel, dim3((384 * 1024 + 255) / 256), dim3(256), 0, s, 1, S, m.I,
-                       (const float*)m.wg_part, grads + m.oU, grads + m.oW, grads + m.ob)))
-    return rc;
+  if (hf) {
+    if ((rc = launch_pdl(wgrad_head_reduce_kernel, dim3(WGR_BLOCKS + HF_BLOCKS), dim3(256), 0, s, 1, S, m.I,
+                         (const float*)m.wg_part, grads + m.oU, grads + m.oW, grads + m.ob, *hf)))
+      return rc;
+  } else {
+    if ((rc = launch_pdl(wgrad_reduce_kernel, dim3(WGR_BLOCKS), dim3(256), 0, s, 1, S, m.I, (const float*)m.wg_part,
+                         grads + m.oU, grads + m.oW, grads + m.ob)))
+      return rc;
+  }
   st.prof->end(LFMQ_REGION_WGRAD, s);
   (void)params;
   (void)c;

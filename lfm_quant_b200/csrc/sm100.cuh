@@ -66,6 +66,16 @@ __device__ __forceinline__ unsigned int ld_acquire_gpu(const unsigned int* p) {
   return v;
 }
 
+// release at gpu scope (cumulative: covers what this thread has observed, e.g. across a preceding bar.sync)
+__device__ __forceinline__ void red_release_gpu_add(unsigned int* p, unsigned int v) {
+  asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+  unsigned long long v;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(v));
+  return v;
+}
+
 // ---- proxies / fences -------------------------------------------------------------------------
 // generic-proxy smem writes -> visible to the async proxy (TMA, tcgen05.mma operand reads)
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
