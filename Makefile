@@ -21,9 +21,3 @@ clean:
 tools: tools/tc_probe
 tools/tc_probe: tools/tc_probe.cu $(CSRC)/sm100.cuh
 	$(NVCC) -O3 -std=c++17 -lineinfo $(ARCH) -o $@ $<
-
-# A/B builds of kernel variants: `make alt ALT_FLAGS="-DLFMQ_BWD_LATE_C0=1"` -> lfm_quant_b200/_lfmq_alt.so (LFMQ_LIB_PATH selects it)
-alt:
-	mkdir -p build/alt
-	for f in lfmq_api kernels_simt lstm_tc rnn_tc; do $(NVCC) $(NVCCFLAGS) $(ALT_FLAGS) -c $(CSRC)/$$f.cu -o build/alt/$$f.o || exit 1; done
-	$(NVCC) $(ARCH) -shared -o lfm_quant_b200/_lfmq_alt.so build/alt/lfmq_api.o build/alt/kernels_simt.o build/alt/lstm_tc.o build/alt/rnn_tc.o -lcudart

@@ -129,7 +129,7 @@ struct TcImpl {
   __nv_bfloat16* dpb;                          // [T][tiles][128][32] bf16 dLoss/dpred tiles (cols >= 16 zero)
   CUtensorMap tm_wos, tm_dpb;
   float* bop;
-  CUtensorMap tm_ubk, tm_px;                   // backward recurrence
+  CUtensorMap tm_ubk;                          // backward recurrence
   CUtensorMap tm_xh_mn, tm_dz_mn;              // weight gradient (MN-major)
   int max_clusters = 0, bwd_max_clusters = 0;
   bool bwd_ready = false;
@@ -225,15 +225,8 @@ constexpr int HP_CSTRIDE = 32;   // head_progress counters one 128-byte line apa
 
 constexpr int FWD_EPI_WARPS = 8;                          // 4 TMEM lane quadrants x 2 column halves
 constexpr int FWD_THREADS = 32 * (2 + FWD_EPI_WARPS);     // producer + MMA + epilogue = 320
-#ifndef LFMQ_FWD_TMA_PUBLISH
-#define LFMQ_FWD_TMA_PUBLISH 0
-#endif
-// Publishing h_t: 0 = a 32-byte STG per thread and chunk followed by a release fence over all of them; 1 = the CTA's
-// [128 x 64] slice staged in shared memory (in the A-operand buffer, which no MMA reads any more once the step's last
-// chunk is committed) and sent as ONE TMA store whose completion is awaited before the peers are signalled.  Measured
-// (profiles/r02_time_c31_fwd_tma_publish.txt): the awaited TMA store takes ~2.5 K cycles under the kernel's own store
-// traffic (580 alone, profiles/r02_micro_tma_store_c30.txt): fwd 0.262 -> 0.315 ms, predict 3.67 -> 4.42 ms.  Off.
-constexpr bool TMA_PUBLISH = LFMQ_FWD_TMA_PUBLISH != 0;
+// h_t is published with one 32-byte STG per thread and chunk; one staged TMA store per CTA was slower
+// (profiles/r02_time_c31_fwd_tma_publish.txt)
 constexpr uint32_t SM_U = 0;                 // 4 k-blocks x [256 x 128 B]
 constexpr uint32_t SM_W = 131072;            // [256 x 64 B]
 constexpr uint32_t SM_H0 = 147456;           // 4 k-blocks x [128 x 128 B]
@@ -255,8 +248,7 @@ struct FwdBars {
 template <bool SAVE>
 __global__ void __launch_bounds__(FWD_THREADS, 1)
     lstm_fwd_tc_kernel(FwdParams p, const __grid_constant__ CUtensorMap tm_h, const __grid_constant__ CUtensorMap tm_x,
-                       const __grid_constant__ CUtensorMap tm_u, const __grid_constant__ CUtensorMap tm_w,
-                       const __grid_constant__ CUtensorMap tm_hst) {
+                       const __grid_constant__ CUtensorMap tm_u, const __grid_constant__ CUtensorMap tm_w) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   FwdBars* bars = reinterpret_cast<FwdBars*>(smem + SM_BARS);
@@ -398,7 +390,6 @@ __global__ void __launch_bounds__(FWD_THREADS, 1)
         const long wblk0 = (((long)t * p.n_tiles_cap + tile_c) * 8 + 2 * (int)rank) * 4 + q;      // jb = 0; jb = 1: + 4
         __nv_bfloat16* grow = SAVE ? p.gates + (wblk0 * 8 * 32 + lane) * 16 + half * 512 : nullptr;   // + gate*1024 (+ jb*4*8*512)
         __nv_bfloat16* crow = SAVE ? p.cst + (wblk0 * 2 * 32 + lane) * 16 + half * 512 : nullptr;     // (+ jb*4*2*512)
-        uint32_t phs[2][8];
 #pragma unroll
         for (int jb = 0; jb < 2; ++jb) {
           const int c = half + 2 * jb;            // 16-unit chunk of this CTA's 64 hidden units
@@ -438,12 +429,7 @@ __global__ void __launch_bounds__(FWD_THREADS, 1)
             pg[jj / 2] = pack_bf16x2(gv[0], gv[1]);
             po[jj / 2] = pack_bf16x2(ov[0], ov[1]);
           }
-          if (TMA_PUBLISH) {
-#pragma unroll
-            for (int e = 0; e < 8; ++e) phs[jb][e] = ph[e];
-          } else if (valid) {
-            st_global_v8(hrow, ph);   // one full 32-byte sector per store (STG.256)
-          }
+          if (valid) st_global_v8(hrow, ph);   // one full 32-byte sector per store (STG.256)
           if (SAVE) {
             // Saved gates / cell states are not needed by the h exchange: park them in the idle accumulator
             // buffer (TMEM) and write them to HBM after the publish, off the per-step critical path.
@@ -458,19 +444,6 @@ __global__ void __launch_bounds__(FWD_THREADS, 1)
             tmem_st_32x32b_x8(tst + 32, cu);
           }
         }
-        if (TMA_PUBLISH) {
-          // all MMAs of the step are complete once chunk 3 is committed: the A-operand buffer is free to stage h_t in
-          // (the peers' multicast of h_t lands there only after every CTA, this one included, has signalled)
-          if (half == 0) mbar_wait(&bars->acc_full[g & 1][3], (g >> 1) & 1);
-          uint8_t* srow = smem + SM_H0 + m * 128;
-#pragma unroll
-          for (int jb = 0; jb < 2; ++jb) {
-            const int ch = (half + 2 * jb) * 2;            // 16-byte chunk of the 128-byte row, 128B-swizzled by row
-            *reinterpret_cast<uint4*>(srow + (((ch) ^ (m & 7)) << 4)) = make_uint4(phs[jb][0], phs[jb][1], phs[jb][2], phs[jb][3]);
-            *reinterpret_cast<uint4*>(srow + (((ch + 1) ^ (m & 7)) << 4)) = make_uint4(phs[jb][4], phs[jb][5], phs[jb][6], phs[jb][7]);
-          }
-          fence_proxy_async_smem();
-        }
         if (SAVE) tmem_st_wait();
         tcgen05_fence_before();
         if (leader) FWD_TRACE(2, t, 1);
@@ -479,14 +452,6 @@ __global__ void __launch_bounds__(FWD_THREADS, 1)
         // Readers acquire at cluster scope and cross into the async proxy before their TMA loads.
         named_bar_sync(1, 32 * FWD_EPI_WARPS);
         if (leader) FWD_TRACE(2, t, 4);
-        if (TMA_PUBLISH && warp == 2) {
-          if (lane == 0) {
-            tma_store_2d(&tm_hst, smem + SM_H0, (t + 1) * TC_XH_LD + (int)rank * TC_HS, tile_c * 128);   // rows >= B clipped
-            bulk_commit_group();
-            bulk_wait_group0();                 // the slice is in global memory before anybody is told
-          }
-          __syncwarp();
-        }
         if (warp == 2 && lane < TC_NC)
           mbar_arrive_cluster(mapa_u32(smem_u32(&bars->h_written), (uint32_t)lane));
         if (SAVE) {
@@ -1788,11 +1753,11 @@ static int tc_run_recurrence(TcState& st, const float* x, int B, bool save, unsi
   p.trace = want_trace ? trace_dev : nullptr;
   if (save) {
     if (int rc = launch_pdl(lstm_fwd_tc_kernel<true>, dim3(TC_NC * p.n_clusters), dim3(FWD_THREADS), FWD_SMEM, s, TC_NC, p,
-                            m.tm_h, m.tm_x, m.tm_u, m.tm_w, m.tm_h128))
+                            m.tm_h, m.tm_x, m.tm_u, m.tm_w))
       return rc;
   } else {
     if (int rc = launch_pdl(lstm_fwd_tc_kernel<false>, dim3(TC_NC * p.n_clusters), dim3(FWD_THREADS), FWD_SMEM, s, TC_NC, p,
-                            m.tm_h, m.tm_x, m.tm_u, m.tm_w, m.tm_h128))
+                            m.tm_h, m.tm_x, m.tm_u, m.tm_w))
       return rc;
   }
   if (want_trace) {
@@ -2008,8 +1973,9 @@ int tc_backward(TcState& st, const lfmq_config& c, const float* params, float* g
 //   keeps them as the A operand in shared memory and multiplies by ITS K-slice of U (resident for the whole unroll):
 //       partial_r[128 x 256] = dz_t[:, own 256 gate cols] * U[all 256 hidden, own gate cols]^T       (tcgen05)
 //   dh_{t-1}[:, slice q] = sum_r partial_r[:, slice q]: the three foreign 128x64 slices travel as bf16 through a
-//   global scratch (written with STG.256, fetched with TMA) -- a reduce-scatter whose volume (48 KB in per CTA and
-//   step) is 5x smaller than all-gathering dz; DSMEM would cost ~3700 cycles for it (profiles/r01_tc_probe.txt).
+//   global scratch (written with STG.256, fetched with one 1-D bulk copy per slice) -- a reduce-scatter whose volume
+//   (48 KB in per CTA and step) is 5x smaller than all-gathering dz; DSMEM would cost ~3700 cycles for it
+//   (profiles/r01_tc_probe.txt).
 //   K order inside the slice: k' = 64*jb + 16*g + jj  <->  gate column g*H + 64r + 16*jb + jj, so hidden chunk jb
 //   (16 units x 4 gates) is one 64-wide k-block and its MMAs overlap the pointwise work of chunk jb+1.
 // =============================================================================================
@@ -2021,7 +1987,7 @@ struct BwdParams {
   const __nv_bfloat16* cst;
   const __nv_bfloat16* dhout;
   __nv_bfloat16* dz;
-  __nv_bfloat16* pexch;      // [tile][parity][src][dst][128][64]
+  __nv_bfloat16* pexch;      // [tile][parity][src][dst][16-column block][128][16]
   long long* trace;          // debug (LFMQ_TRACE_BWD=1)
   unsigned long long* progress;   // null, or where CTA 0 publishes base + (steps it has completed)
   unsigned long long base;
@@ -2033,39 +1999,12 @@ struct BwdParams {
   } while (0)
 
 constexpr int BWD_NC = 4;
-#ifndef LFMQ_BWD_LATE_C1
-#define LFMQ_BWD_LATE_C1 1
-#endif
-constexpr bool LATE_C1 = LFMQ_BWD_LATE_C1 == 1;     // at the top of the step
-constexpr bool POST_C1 = LFMQ_BWD_LATE_C1 == 2;     // experiment: right after the export stores of the previous step
-#ifndef LFMQ_BWD_LATE_C0
-#define LFMQ_BWD_LATE_C0 0
-#endif
-#ifndef LFMQ_BWD_DSMEM
-#define LFMQ_BWD_DSMEM 0
-#endif
-// Partial exchange: 0 = through L2 (st.global, cluster arrive, TMA load by the peer's producer); 1 = every pointwise
-// thread pushes its piece of the foreign slices straight into the peers' shared memory (st.async completing tx-bytes on
-// the peer's recv_full).  Measured (profiles/r02_time_c19_dsmem_exchange.txt): the push makes the export itself shorter
-// (3.4 K -> 1.9 K cycles) but the 48 KB per CTA and step take ~4 K cycles to land (DSMEM moves ~12 B/clk/SM), against
-// 2.6 K for signal + TMA load from L2: bwd 0.304 -> 0.341 ms.  Kept as a build option, off.
-constexpr bool DSMEM_X = LFMQ_BWD_DSMEM != 0;
-#ifndef LFMQ_BWD_WARP_SIGNAL
-#define LFMQ_BWD_WARP_SIGNAL 0
-#endif
-// 1 = every pointwise warp signals the peers itself after its own export stores (no CTA-wide named barrier first)
-constexpr bool WARP_SIG = LFMQ_BWD_WARP_SIGNAL != 0 && !DSMEM_X;
-#ifndef LFMQ_BWD_EXPORT_BATCH
-#define LFMQ_BWD_EXPORT_BATCH 1
-#endif
-constexpr bool EXPORT_BATCH = LFMQ_BWD_EXPORT_BATCH != 0;
-#ifndef LFMQ_BWD_PX_BLOCKED
-#define LFMQ_BWD_PX_BLOCKED 1
-#endif
-// exchange scratch as [16-column block][row][16]: a warp's 256-bit export store is 1 KB contiguous (it was 32 separate
-// 32-byte pieces, one per 128-byte row), the receiver fetches its 16 KB slice with one 1-D bulk copy and reads it as is
-constexpr bool PX_BLOCKED = LFMQ_BWD_PX_BLOCKED != 0 && !DSMEM_X;
-constexpr bool LATE_C0 = LFMQ_BWD_LATE_C0 != 0;     // experiment: the first chunk's operands at the top of the step as well
+// Partial exchange through L2: st.global of the foreign slices, a cluster arrive, one 1-D bulk copy per slice by the
+// peer's producer.  The exchange scratch is [16-column block][row][16], so a warp's 256-bit export store is 1 KB
+// contiguous and the receiver reads its 16 KB slice as it lands.  Rejected alternatives, measured on a B200:
+//   pushing the slices into the peers' shared memory with st.async: profiles/r02_time_c19_dsmem_exchange.txt
+//   a row-major scratch fetched with a 2-D TMA load: profiles/r02_time_c26_blocked_exchange.txt
+//   per-warp peer signalling, next operands after the export: profiles/r02_time_c20_bwd_variants.txt
 // Warp roles, by warpgroup (setmaxnreg moves registers between warpgroups): warps 0-3 pointwise set 0, warps 4-7 pointwise
 // set 1, warps 8-11 = producer, MMA issuer, dz store, idle.  The role warpgroup gives its registers up (72 each), the
 // pointwise warps take 216 (2 x 216 + 72 = the 504 of the 168 x 3 pool): the 168 of an even split left ~100 spilled values on the pointwise warps' path, with next to
@@ -2091,8 +2030,7 @@ struct BwdBars {
 // step on the 8 KB dpred tile) into the accumulator whose own slice the pointwise warps read anyway.
 template <bool FUSED>
 __global__ void __launch_bounds__(BWD_THREADS, 1)
-    lstm_bwd_tc_kernel(BwdParams p, const __grid_constant__ CUtensorMap tm_ubk,
-                       const __grid_constant__ CUtensorMap tm_px, const __grid_constant__ CUtensorMap tm_dzst,
+    lstm_bwd_tc_kernel(BwdParams p, const __grid_constant__ CUtensorMap tm_ubk, const __grid_constant__ CUtensorMap tm_dzst,
                        const __grid_constant__ CUtensorMap tm_dpb, const __grid_constant__ CUtensorMap tm_wos) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -2110,8 +2048,8 @@ __global__ void __launch_bounds__(BWD_THREADS, 1)
       mbar_init(&bars->acc_full[i], 1);
     }
     mbar_init(&bars->recv_full, 1);
-    mbar_init(&bars->recv_free, WARP_SIG ? 8 : 1);
-    mbar_init(&bars->exp_ready, (DSMEM_X || WARP_SIG) ? (BWD_NC - 1) * 8 : BWD_NC - 1);   // DSMEM_X: 'peers have read my last export'
+    mbar_init(&bars->recv_free, 1);
+    mbar_init(&bars->exp_ready, BWD_NC - 1);   // one arrival per peer: its export for this CTA is in global memory
     mbar_init(&bars->dpb_full, 1);
     mbar_init(&bars->dpb_free, 1);
     fence_mbar_init();
@@ -2150,13 +2088,7 @@ __global__ void __launch_bounds__(BWD_THREADS, 1)
       if (FUSED && lane == 0) load_dpred(tile, T - 1);
       for (int t = T - 1; t >= 0; --t) {
         if (FUSED && lane == 0 && t > 0) load_dpred(tile, t - 1);      // for the MMA appended to this step
-        if (DSMEM_X && lane == 0 && t <= T - 2) {    // peers push the slices themselves: only arm the barrier, one phase
-          if (n_er > 0) mbar_wait(&bars->recv_full, (n_er - 1) & 1);    // at a time
-          ++n_er;
-          BWD_TRACE(0, T - 1 - t, 0);
-          mbar_arrive_expect_tx(&bars->recv_full, 3 * 16384);
-        }
-        if (!DSMEM_X && lane == 0 && t <= T - 2) {   // step t consumes the partials exported after step t+1
+        if (lane == 0 && t <= T - 2) {   // step t consumes the partials exported after step t+1
           mbar_wait_cluster(&bars->exp_ready, (n_er) & 1);
           mbar_wait(&bars->recv_free, (n_er++) & 1);    // own epilogue is done reading the previous slices
           BWD_TRACE(0, T - 1 - t, 0);
@@ -2165,13 +2097,9 @@ __global__ void __launch_bounds__(BWD_THREADS, 1)
           const int par = (t + 1) & 1;
           for (uint32_t d = 1; d < BWD_NC; ++d) {
             const uint32_t src = (rank + d) & 3;
-            if (PX_BLOCKED)
-              bulk_load_1d(smem + SB_R + (d - 1) * 16384,
-                           p.pexch + ((((long)(tile * 2 + par) * 4 + (int)src) * 4 + (int)rank)) * 128 * 64, 16384,
-                           &bars->recv_full);
-            else
-              tma_load_2d(smem + SB_R + (d - 1) * 16384, &tm_px, &bars->recv_full, 0,
-                          ((((tile * 2 + par) * 4 + (int)src) * 4 + (int)rank)) * 128);
+            bulk_load_1d(smem + SB_R + (d - 1) * 16384,
+                         p.pexch + ((((long)(tile * 2 + par) * 4 + (int)src) * 4 + (int)rank)) * 128 * 64, 16384,
+                         &bars->recv_full);
           }
         }
         __syncwarp();
@@ -2267,7 +2195,6 @@ __global__ void __launch_bounds__(BWD_THREADS, 1)
     const int sw = m & 7;
     float dc[32];
     uint32_t gs = 0, n_rf = 0;
-    uint32_t n_exp = 0;                      // exports done (DSMEM_X)
     uint32_t caf[2] = {0, 0};                // completed phases of acc_full[b] (mirrors the MMA warp's commit sequence)
     // inputs of this set's two chunks of one step (slot ci): loaded ahead of the exchange they do not depend on
     uint32_t gi[2][8], gf[2][8], gg[2][8], go[2][8], dhp[2][8], ct[2][8], cp[2][8];
@@ -2313,8 +2240,7 @@ __global__ void __launch_bounds__(BWD_THREADS, 1)
       const bool valid = b < p.B;
 #pragma unroll
       for (int j = 0; j < 32; ++j) dc[j] = 0.f;
-      if (!LATE_C0) load_chunk(0, tile, valid, T - 1);
-      if (!LATE_C1) load_chunk(1, tile, valid, T - 1);     // (also POST_C1: nothing precedes the first step)
+      load_chunk(0, tile, valid, T - 1);
       if (FUSED) {                             // the head's dLoss/dh_{T-1} for the own slice is in the accumulator
         const uint32_t pb = (gs + 1) & 1;
         mbar_wait(&bars->acc_full[pb], caf[pb] & 1);
@@ -2323,10 +2249,10 @@ __global__ void __launch_bounds__(BWD_THREADS, 1)
       for (int t = T - 1; t >= 0; --t, ++gs) {
         const bool has_rec = t < T - 1;
         const uint32_t acc_prev = tmem + ((gs + 1) & 1) * 256;     // partial of step t+1 (own slice still there)
-        // LATE_C1: the second chunk's operands are requested only now and land under the first chunk's arithmetic, so
-        // that only one chunk's operands (48 registers, not 96) are live across the export section below
-        if (LATE_C0) load_chunk(0, tile, valid, t);
-        if (LATE_C1) load_chunk(1, tile, valid, t);
+        // the second chunk's operands are requested only now and land under the first chunk's arithmetic, so that only
+        // one chunk's operands (48 registers, not 96) are live across the export section below (one step ahead, or the
+        // first chunk's here as well, were slower: profiles/r02_summary.md, c15/c16 and c18)
+        load_chunk(1, tile, valid, t);
         if (has_rec) mbar_wait(&bars->recv_full, (n_rf++) & 1);
         if (tid == 64) BWD_TRACE(2, T - 1 - t, 0);
 #pragma unroll
@@ -2342,10 +2268,10 @@ __global__ void __launch_bounds__(BWD_THREADS, 1)
             for (int j = 0; j < 16; ++j) rec[j] = __uint_as_float(vr[j]);
 #pragma unroll
             for (int d = 0; d < 3 && has_rec; ++d) {
-              const uint8_t* rs = smem + SB_R + d * 16384 + (PX_BLOCKED ? (jb * 128 + m) * 32 : m * 128);
+              const uint8_t* rs = smem + SB_R + d * 16384 + (jb * 128 + m) * 32;
 #pragma unroll
               for (int h2 = 0; h2 < 2; ++h2) {
-                const uint4 v = *reinterpret_cast<const uint4*>(rs + (PX_BLOCKED ? h2 << 4 : ((2 * jb + h2) ^ sw) << 4));
+                const uint4 v = *reinterpret_cast<const uint4*>(rs + (h2 << 4));
                 const uint32_t w[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
@@ -2402,19 +2328,11 @@ __global__ void __launch_bounds__(BWD_THREADS, 1)
           if (tid == 192 && ci == 0) BWD_TRACE(0, T - 1 - t, 1);     // warp-set 1 in the producer row's free slots
           if (tid == 192 && ci == 1) BWD_TRACE(0, T - 1 - t, 2);
         }
-        if (DSMEM_X && has_rec) {                    // this warp is done with the received slices: tell the three senders
-          __syncwarp();
-          if (lane >= 1 && lane < BWD_NC)
-            mbar_arrive_cluster(mapa_u32(smem_u32(&bars->exp_ready), (rank + (uint32_t)lane) & 3));
-        }
-        // inputs of both chunks of the next step: independent of the exchange below.  Placement matters because the
+        // inputs of the next step's first chunk: independent of the exchange below.  Placement matters because the
         // SM's memory pipe is a FIFO: issued here they delay the export slightly but land before the next step
         // starts; issued after the export they arrive too late (+9 % kernel time), issued inside the chunk loop they
         // hold up the chunk's own dz / A-operand stores (+17 %).
-        if (t > 0) {
-          if (!LATE_C0) load_chunk(0, tile, valid, t - 1);
-          if (!LATE_C1 && !POST_C1) load_chunk(1, tile, valid, t - 1);
-        }
+        if (t > 0) load_chunk(0, tile, valid, t - 1);
         // ---- export the foreign slices of partial_t (needed by the peers for step t-1) ----
         if (t > 0) {
           mbar_wait(&bars->acc_full[gs & 1], caf[gs & 1] & 1);
@@ -2422,80 +2340,37 @@ __global__ void __launch_bounds__(BWD_THREADS, 1)
           tcgen05_fence_after();
           const uint32_t acc = tmem + (gs & 1) * 256 + lane_addr;
           const int par = t & 1;
-          if (DSMEM_X) {
-            // all 24 reader warps of the three peers have released the slices of the previous export
-            if (n_exp > 0) mbar_wait_cluster(&bars->exp_ready, (n_exp - 1) & 1);
-            ++n_exp;
+          // all six 16-column pieces requested from TMEM before the first is waited for: one tcgen05.ld latency
+          // instead of six (the 216-register budget of the pointwise warpgroups has room for the 96 values)
+          uint32_t v[6][16];
 #pragma unroll
-            for (uint32_t d = 1; d < BWD_NC; ++d) {
-              const uint32_t dst = (rank + d) & 3;
-              // at the receiver, slot (d' - 1) holds the slice of source (dst + d') & 3: d' = 4 - d
-              const uint32_t rrow = mapa_u32(smem_u32(smem + SB_R + (3 - d) * 16384 + m * 128), dst);
-              const uint32_t rbar = mapa_u32(smem_u32(&bars->recv_full), dst);
+          for (uint32_t d = 1; d < BWD_NC; ++d)
 #pragma unroll
-              for (int hh = 0; hh < 2; ++hh) {
-                uint32_t v[16];
-                tmem_ld_32x32b_x16(acc + dst * 64 + set * 32 + hh * 16, v);
-                tmem_ld_wait();
-                uint32_t pk[8];
+            for (int hh = 0; hh < 2; ++hh)
+              tmem_ld_32x32b_x16(acc + ((rank + d) & 3) * 64 + set * 32 + hh * 16, v[(d - 1) * 2 + hh]);
+          tmem_ld_wait();
 #pragma unroll
-                for (int e = 0; e < 8; ++e) pk[e] = pack_bf16x2(__uint_as_float(v[2 * e]), __uint_as_float(v[2 * e + 1]));
-                const int c0 = set * 4 + hh * 2;           // 16-byte chunk of the 64-column slice, 128B-swizzled by row
-                st_async_v4(rrow + (((c0) ^ sw) << 4), rbar, pk[0], pk[1], pk[2], pk[3]);
-                st_async_v4(rrow + (((c0 + 1) ^ sw) << 4), rbar, pk[4], pk[5], pk[6], pk[7]);
-              }
-            }
-          }
-#pragma unroll
-          if (!DSMEM_X && EXPORT_BATCH) {
-            // all six 16-column pieces requested from TMEM before the first is waited for: one tcgen05.ld latency
-            // instead of six (the 216-register budget of the pointwise warpgroups has room for the 96 values)
-            uint32_t v[6][16];
-#pragma unroll
-            for (uint32_t d = 1; d < BWD_NC; ++d)
-#pragma unroll
-              for (int hh = 0; hh < 2; ++hh)
-                tmem_ld_32x32b_x16(acc + ((rank + d) & 3) * 64 + set * 32 + hh * 16, v[(d - 1) * 2 + hh]);
-            tmem_ld_wait();
-#pragma unroll
-            for (uint32_t d = 1; d < BWD_NC; ++d) {
-              const uint32_t dst = (rank + d) & 3;
-              __nv_bfloat16* slice = p.pexch + (((long)(tile * 2 + par) * 4 + rank) * 4 + dst) * 128 * 64;
-              __nv_bfloat16* out = PX_BLOCKED ? slice + ((long)(set * 2) * 128 + m) * 16 : slice + m * 64 + set * 32;
-#pragma unroll
-              for (int hh = 0; hh < 2; ++hh) {
-                const uint32_t* vv = v[(d - 1) * 2 + hh];
-                uint32_t pk[8];
-#pragma unroll
-                for (int e = 0; e < 8; ++e) pk[e] = pack_bf16x2(__uint_as_float(vv[2 * e]), __uint_as_float(vv[2 * e + 1]));
-                st_global_v8(out + hh * (PX_BLOCKED ? 128 * 16 : 16), pk);
-              }
-            }
-          }
-#pragma unroll
-          for (uint32_t d = 1; d < BWD_NC && !DSMEM_X && !EXPORT_BATCH; ++d) {
+          for (uint32_t d = 1; d < BWD_NC; ++d) {
             const uint32_t dst = (rank + d) & 3;
             __nv_bfloat16* slice = p.pexch + (((long)(tile * 2 + par) * 4 + rank) * 4 + dst) * 128 * 64;
-            __nv_bfloat16* out = PX_BLOCKED ? slice + ((long)(set * 2) * 128 + m) * 16 : slice + m * 64 + set * 32;
+            __nv_bfloat16* out = slice + ((long)(set * 2) * 128 + m) * 16;
 #pragma unroll
             for (int hh = 0; hh < 2; ++hh) {
-              uint32_t v[16];
-              tmem_ld_32x32b_x16(acc + dst * 64 + set * 32 + hh * 16, v);
-              tmem_ld_wait();
+              const uint32_t* vv = v[(d - 1) * 2 + hh];
               uint32_t pk[8];
 #pragma unroll
-              for (int e = 0; e < 8; ++e) pk[e] = pack_bf16x2(__uint_as_float(v[2 * e]), __uint_as_float(v[2 * e + 1]));
-              st_global_v8(out + hh * (PX_BLOCKED ? 128 * 16 : 16), pk);
+              for (int e = 0; e < 8; ++e) pk[e] = pack_bf16x2(__uint_as_float(vv[2 * e]), __uint_as_float(vv[2 * e + 1]));
+              st_global_v8(out + hh * 128 * 16, pk);
             }
           }
           tcgen05_fence_before();
-          if (POST_C1) load_chunk(1, tile, valid, t - 1);
           if (tid == 64) BWD_TRACE(2, T - 1 - t, 4);
-          if (!DSMEM_X && !WARP_SIG) named_bar_sync(1, 256);
-          if (WARP_SIG) __syncwarp();
+          // all 256 pointwise threads have read the received slices and stored their export: warp 0 frees the receive
+          // buffer for the own producer and tells the three peers
+          named_bar_sync(1, 256);
           if (tid == 64) BWD_TRACE(2, T - 1 - t, 5);
-          if (!DSMEM_X && (warp == 0 || WARP_SIG) && lane == 0) mbar_arrive(&bars->recv_free);
-          if (!DSMEM_X && (warp == 0 || WARP_SIG) && lane >= 1 && lane < BWD_NC) {
+          if (warp == 0 && lane == 0) mbar_arrive(&bars->recv_free);
+          if (warp == 0 && lane >= 1 && lane < BWD_NC) {
             mbar_arrive_cluster(mapa_u32(smem_u32(&bars->exp_ready), (rank + (uint32_t)lane) & 3));
           }
         }
@@ -2700,8 +2575,6 @@ int tc_backward_impl(TcState& st, const lfmq_config& c, const float* params, flo
     LFMQ_CUDA_CHECK(cudaFuncSetAttribute(lstm_bwd_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM));
     LFMQ_CUDA_CHECK(cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WG_SMEM));
     if ((rc = make_map_2d(&m.tm_ubk, m.Ubk, 256, 4 * TC_H, 512, 64, 256, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-    const uint64_t px_rows = (uint64_t)((m.maxB + 127) / 128) * 2 * 16 * 128;
-    if ((rc = make_map_2d(&m.tm_px, m.pexch, 64, px_rows, 128, 64, 128, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
     cudaLaunchConfig_t qc = {};
     qc.gridDim = dim3(BWD_NC * 37);
     qc.blockDim = dim3(BWD_THREADS);
@@ -2770,11 +2643,11 @@ int tc_backward_impl(TcState& st, const lfmq_config& c, const float* params, flo
     }
     if (fused) {
       if ((rc = launch_pdl(lstm_bwd_tc_kernel<true>, dim3(BWD_NC * bp.n_clusters), dim3(BWD_THREADS), BWD_SMEM, s, BWD_NC, bp,
-                           m.tm_ubk, m.tm_px, tm_dzst, m.tm_dpb, m.tm_wos)))
+                           m.tm_ubk, tm_dzst, m.tm_dpb, m.tm_wos)))
         return rc;
     } else {
       if ((rc = launch_pdl(lstm_bwd_tc_kernel<false>, dim3(BWD_NC * bp.n_clusters), dim3(BWD_THREADS), BWD_SMEM, s, BWD_NC, bp,
-                           m.tm_ubk, m.tm_px, tm_dzst, m.tm_dpb, m.tm_wos)))
+                           m.tm_ubk, tm_dzst, m.tm_dpb, m.tm_wos)))
         return rc;
     }
     if (pf_lead > 0) LFMQ_CUDA_CHECK(cudaStreamWaitEvent(s, m.ev_join, 0));

@@ -103,9 +103,6 @@ struct GArgs {
   unsigned int* gbar;  // [gridDim.x], zeroed before the launch; counts the group's CTAs that have finished a step
 };
 
-#ifndef LFMQ_GEN_BWD_EW
-#define LFMQ_GEN_BWD_EW 2
-#endif
 enum { EPI_FWD = 0, EPI_BWD = 1, EPI_STORE = 2, EPI_FWD_ACC = 3, EPI_HEAD = 4 };   // _ACC: expf / tanhf (bf16x3)
 
 struct EpiParams {
@@ -150,18 +147,13 @@ struct EpiParams {
 // CTAs leave: the loads are latency-bound (~5 K cycles per stage under load), bytes in flight are what buys bandwidth.
 template <int BN, int MT, int EPI = 0>
 struct GSmem {
-  static constexpr int EW = (EPI == 1) ? LFMQ_GEN_BWD_EW : 1;   // warps per TMEM lane quadrant and M tile (EPI_BWD)
+  static constexpr int EW = (EPI == 1) ? 2 : 1;   // warps per TMEM lane quadrant and M tile (EPI_BWD)
   static constexpr uint32_t A_BYTES = MT * 128 * 128;     // MT x (128 rows x 64 bf16)
   static constexpr uint32_t B_BYTES = BN * 128;
   static constexpr uint32_t STAGE = A_BYTES + B_BYTES;
   // one launch = one wave for the recurrence steps (<= 148 tiles: one CTA per SM, deep ring); the multi-wave GEMMs keep
   // two CTAs per SM
-#ifndef LFMQ_GEN_BWD_2CTA
-#define LFMQ_GEN_BWD_2CTA 0
-#endif
-  // (LFMQ_GEN_BWD_2CTA: experiment -- two 64-unit backward CTAs per SM so that one's epilogue can overlap the other's mainloop)
-  static constexpr int CTAS_PER_SM =
-      (MT == 1 && (BN >= 256 || EPI == 2 || EPI == 4 || (LFMQ_GEN_BWD_2CTA && EPI == 1 && BN == 64))) ? 2 : 1;      // (2 = EPI_STORE, 4 = EPI_HEAD)
+  static constexpr int CTAS_PER_SM = (MT == 1 && (BN >= 256 || EPI == 2 || EPI == 4)) ? 2 : 1;   // (2 = EPI_STORE, 4 = EPI_HEAD)
   static constexpr int NS = (int)((CTAS_PER_SM == 2 ? 98304u : 196608u) / STAGE);
   static constexpr uint32_t BARS = NS * STAGE;
   static constexpr uint32_t TOTAL = BARS + 256 + 1024;    // + alignment slack
@@ -1425,11 +1417,7 @@ void gen_layout(GenState& st, const lfmq_config& c, const GenLayerOff* lo, int64
   m.x3 = c.precision == LFMQ_PREC_BF16X3;
   m.train_ws = !c.forward_only;
   m.oWo = oWo; m.obo = obo;
-  m.BNU = (m.H % 128 == 0) ? 128 : 64;
-  {   // experiment (LFMQ_GEN_BWD_BN64=1): 64-unit backward tiles also when H % 128 == 0 -> twice the CTAs per step
-    static const char* e = getenv("LFMQ_GEN_BWD_BN64");
-    if (e && atoi(e)) m.BNU = 64;
-  }
+  m.BNU = (m.H % 128 == 0) ? 128 : 64;   // 64-unit tiles at H % 128 == 0 were slower (profiles/r02_summary.md, c28)
   const size_t T = m.T, Bp = m.Bp, H = m.H;
   const bool rec = (c.train && c.recurrent_dropout > 0.f);
   m.layers.assign(m.L, GenLayer{});

@@ -104,15 +104,6 @@ __device__ __forceinline__ void st_cluster_v4(uint32_t addr, uint32_t a, uint32_
                : "memory");
 }
 
-// 16 B into a peer CTA's shared memory, completing 16 tx-bytes on a barrier of that same peer (no fence, no arrive needed)
-__device__ __forceinline__ void st_async_v4(uint32_t remote_addr, uint32_t remote_bar, uint32_t a, uint32_t b, uint32_t c,
-                                            uint32_t d) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];" ::"r"(
-                   remote_addr),
-               "r"(a), "r"(b), "r"(c), "r"(d), "r"(remote_bar)
-               : "memory");
-}
-
 // ---- TMA --------------------------------------------------------------------------------------
 __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* m) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(m)) : "memory");
